@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference's numpy CPU path (oracle port)
+    python bench.py --dump-outputs DIR ...    # also write sampled signature rows to DIR/*.npy (see dump_rows)
 
 A "step" is one pass of the hot path over one batch of synthetic token hashes.
   value  : whole-job signatures/s with inputs already resident in HBM (CUDA events on the
@@ -55,7 +56,25 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-dups", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed sample of rows of each timed signature matrix (rank 0) "
+                         "to DIR/<name>.npy as float64, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what this project's GPU path computed: it needs --impl ours")
+    return args
+
+
+DUMP_BYTES = 63_000_000   # array bytes --dump-outputs writes at most: under 64 MB in all with the .npy headers
+
+
+def dump_rows(n_docs: int, k: int) -> np.ndarray:
+    """Sorted indices of the rows that --dump-outputs writes of each signature matrix (up to three matrices of
+    float64): every row when they fit, else a seeded sample that depends on --docs and --num-perm only."""
+    m = min(n_docs, DUMP_BYTES // (8 * (3 * k + 1)))
+    return np.sort(np.random.default_rng(0).choice(n_docs, size=m, replace=False))
 
 
 # ---------------------------------------------------------------------------------------------
@@ -72,10 +91,10 @@ def make_tokens(n_docs: int, t: int, seed: int, out: np.ndarray) -> None:
 
 
 # ---------------------------------------------------------------------------------------------
-# CPU baseline: the reference's own MinHash.bulk when baseline/_ref holds the reference install
-# (tools/install_reference.sh), else the oracle port of its numpy path; all host cores, pinned workers
+# CPU baseline: the reference's own MinHash.bulk when oracle/_ref/site holds the reference install
+# (oracle/stage_reference.sh, run by build()), else the oracle port of its numpy path; all host cores, pinned workers
 # ---------------------------------------------------------------------------------------------
-REF_DIR = os.path.join(ROOT, "baseline", "_ref")
+REF_DIR = os.path.join(ROOT, "oracle", "_ref", "site")
 
 
 def reference_kind() -> str:
@@ -157,7 +176,7 @@ def workload_config(args, cores: int) -> dict:
 
 
 def cpu_sample_text(sample: int, t: int, cores: int, kind: str, rates) -> str:
-    what = ("datasketch.MinHash.bulk (the unmodified reference from baseline/_ref, hashfunc=identity on pre-hashed tokens)"
+    what = ("datasketch.MinHash.bulk (the unmodified reference from oracle/_ref/site, hashfunc=identity on pre-hashed tokens)"
             if kind == "reference" else "oracle port of datasketch's numpy uint64 path")
     return ("%d docs x %d tokens per repeat, best of %d repeats (%s sig/s), %s over %d pinned processes"
             % (sample, t, len(rates), "/".join("%.0f" % r for r in rates), what, cores))
@@ -240,8 +259,8 @@ def bind_to_gpu_numa_node(gpu_index: int):
 # ---------------------------------------------------------------------------------------------
 def run_reference(args):
     """--impl reference: the reference's own CPU implementation of the path -- datasketch.MinHash.bulk from
-    baseline/_ref when installed (kind "reference"), else its numpy uint64 arithmetic restated in
-    oracle/oracle_np.py (kind "port"; /root/reference is absent on the GPU box) -- on all host cores;
+    oracle/_ref/site when installed (kind "reference"), else its numpy uint64 arithmetic restated in
+    oracle/oracle_np.py (kind "port", where no reference was staged) -- on all host cores;
     each step = a bounded sample of the same workload."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -362,6 +381,17 @@ def run_ours(args):
     ms_step = ms_total / args.steps
     value = n * world / (ms_step * 1e-3)
 
+    # --dump-outputs: the sampled rows of what each timed leg's last step wrote, taken before the next leg runs
+    dump = bool(args.dump_outputs) and rank == 0
+    dumped = {}
+    if dump:
+        rows = dump_rows(n, k)
+        d_rows = torch.from_numpy(rows).to(dev)
+
+        def take(name, sig):
+            dumped[name] = sig[d_rows].cpu().numpy().view(np.uint32).astype(np.float64)
+        take("signatures", d_out)
+
     # parity spot-check on the benchmark's own output, on EVERY rank (oracle = checker only)
     from oracle import oracle_clib as oc
     idx = np.arange(0, n, max(1, n // 64))[:64]
@@ -399,6 +429,8 @@ def run_ours(args):
         ev1.record(stream)
         barrier()
         ms_d = ev0.elapsed_time(ev1) / args.steps
+        if dump:
+            take("signatures_repeats", d_out2)
         sub_d = d_dup.view(n, t)[torch.from_numpy(idx).to(dev)].cpu().numpy().view(np.uint32).reshape(-1)
         want_d = oc.minhash_bulk_u32tok(np.ascontiguousarray(sub_d), np.arange(len(idx) + 1, dtype=np.int64) * t, perms)
         if not np.array_equal(d_out2[torch.from_numpy(idx).to(dev)].cpu().numpy().view(np.uint32), want_d):
@@ -418,18 +450,20 @@ def run_ours(args):
         d_tok64.mul_(1 << 32).add_(d_tok.view(-1).to(torch.int64) & 0xFFFFFFFF)   # (hi << 32) | lo, as the bit pattern
         d_out3 = torch.empty_like(d_out)
         res = {}
-        for name, steps in (("two_phase", args.steps), ("exact", min(args.steps, 3))):
+        for name in ("two_phase", "exact"):
             def step64():
                 dsk.engine.bulk_signatures_device(d_tok64, d_off, n * t, perms, d_out=d_out3, kernel=name, stream=stream.cuda_stream)
             for _ in range(2):
                 step64()
             barrier()
             ev0.record(stream)
-            for _ in range(steps):
+            for _ in range(args.steps):
                 step64()
             ev1.record(stream)
             barrier()
-            res[name] = ev0.elapsed_time(ev1) / steps
+            res[name] = ev0.elapsed_time(ev1) / args.steps
+            if dump and name == "two_phase":
+                take("signatures_u64", d_out3)
             sub64 = d_tok64.view(n, t)[torch.from_numpy(idx).to(dev)].cpu().numpy().view(np.uint64).reshape(-1)
             want64 = oc.minhash_bulk_u64tok(np.ascontiguousarray(sub64), np.arange(len(idx) + 1, dtype=np.int64) * t, perms)
             if not np.array_equal(d_out3[torch.from_numpy(idx).to(dev)].cpu().numpy().view(np.uint32), want64):
@@ -437,7 +471,7 @@ def run_ours(args):
         u64_tokens = {"ms_per_step": res["two_phase"], "value": n / (res["two_phase"] * 1e-3), "unit": UNIT + " per GPU",
                       "slowdown_vs_u32": res["two_phase"] / ms_step, "exact_kernel_ms_per_step": res["exact"],
                       "speedup_vs_exact_kernel": res["exact"] / res["two_phase"], "rows_verified": True,
-                      "steps": {"two_phase": args.steps, "exact": min(args.steps, 3)}}
+                      "steps": {"two_phase": args.steps, "exact": args.steps}}
         del d_tok64, d_out3
 
     # ---- e2e: pinned host buffers through the host C-ABI ------------------------------------------
@@ -655,7 +689,7 @@ def run_ours(args):
             # the two-phase path launches minhash_sig_kernel twice per device-resident step (documents, then the piece
             # table of long documents -- empty here, an idle launch); the host pipeline launches it once per slice
             "gpu_launches": (2 if kern == "two_phase" else 1) * args.steps * (1 if duplicates is None else 2) + e2e_launches
-                            + (0 if u64_tokens is None else 2 * args.steps + min(args.steps, 3)),
+                            + (0 if u64_tokens is None else 3 * args.steps),
         }
         # the roof that actually binds this kernel: one 32-bit IMAD per (token, permutation) evaluation is the floor
         # of any exact scheme, and B200 issues IMAD at 16 lanes/clk/SMSP = 64 lanes/clk/SM (profiles/, DESIGN.md 5)
@@ -676,6 +710,11 @@ def run_ours(args):
         if u64_tokens is not None:
             line["u64_tokens"] = u64_tokens
         print(json.dumps(line), flush=True)
+    if dump:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        dumped["rows"] = rows.astype(np.float64)
+        for name, arr in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     if world > 1:
         dist.destroy_process_group()
 

@@ -1,13 +1,12 @@
 """The reference's OWN unittest files, run against datasketch_b200 on the GPU -- the drop-in gate.
 
-``tools/make_refcheck.sh`` stages ekzhu/datasketch's ``test/test_minhash.py``, ``test_lean_minhash.py``,
-``test_weighted_minhash.py``, ``test_lsh.py``, ``test_lshforest.py``, ``test_lshensemble.py`` and ``test_lshbloom.py``
-next to an import shim (``datasketch`` -> ``datasketch_b200``) in the git-ignored ``_refcheck/``; the staging happens in
-the build container (where ``/root/reference`` exists) and the directory travels to the GPU box with the snapshot.  Here
-the files run unchanged in a subprocess against the real library.  Deselected: the Redis-backed cases (storage backends
-are out of scope; the shim's ``mockredis`` raises SkipTest).  If neither the staged directory nor a reference checkout
-is present the test is SKIPPED with that reason -- it never passes vacuously.
-Reference: /root/reference/test/test_minhash.py:109-124, test_lsh.py:109-125 and the rest of those files.
+``oracle/stage_reference.sh`` (run by ``build()`` where a reference checkout is readable) stages ekzhu/datasketch's
+``test/test_minhash.py``, ``test_lean_minhash.py``, ``test_weighted_minhash.py``, ``test_lsh.py``, ``test_lshforest.py``,
+``test_lshensemble.py`` and ``test_lshbloom.py`` next to an import shim (``datasketch`` -> ``datasketch_b200``) in the
+git-ignored ``oracle/_ref/refcheck/``, which a built tree carries along.  Here the files run unchanged in a subprocess
+against the real library.  Deselected: the Redis-backed cases (storage backends are out of scope; the shim's
+``mockredis`` raises SkipTest).  Without the staged files the test is SKIPPED with that reason -- it never passes
+vacuously; ``tests/test_api_behaviour.py`` is the self-contained comparison with the reference.
 """
 import os
 import subprocess
@@ -16,8 +15,7 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("DATASKETCH_REF", "/root/reference")
-STAGE = os.path.join(ROOT, "_refcheck")
+STAGE = os.path.join(ROOT, "oracle", "_ref", "refcheck")
 FILES = ["test_minhash.py", "test_lean_minhash.py", "test_weighted_minhash.py", "test_lsh.py", "test_lshforest.py",
          "test_lshensemble.py", "test_lshbloom.py"]
 
@@ -25,10 +23,8 @@ FILES = ["test_minhash.py", "test_lean_minhash.py", "test_weighted_minhash.py", 
 @pytest.mark.gpu
 def test_reference_unittests_pass_on_the_gpu(tmp_path):
     if not os.path.isdir(os.path.join(STAGE, "test")):
-        if not os.path.isdir(os.path.join(REF, "test")):
-            pytest.skip("the reference's test files are not staged (_refcheck/ absent: run tools/make_refcheck.sh in the "
-                        "build container) and no reference checkout exists at %s" % REF)
-        subprocess.run(["bash", os.path.join(ROOT, "tools", "make_refcheck.sh")], check=True, capture_output=True)
+        pytest.skip("the reference's test files are not staged (oracle/_ref/refcheck/ absent: build() stages them "
+                    "where a reference checkout is readable, see oracle/stage_reference.sh)")
     files = [os.path.join(STAGE, "test", f) for f in FILES if os.path.exists(os.path.join(STAGE, "test", f))]
     assert len(files) == len(FILES), files
     env = dict(os.environ, PYTHONPATH=os.pathsep.join([STAGE, ROOT, os.environ.get("PYTHONPATH", "")]))
