@@ -26,6 +26,9 @@
 
 namespace dsk {
 
+// dynamic shared memory one block may opt in to on sm_100 (227 KB); launchers size their tiles against it
+constexpr size_t kMaxDynamicSmemPerBlock = 232448;
+
 // ---- thread-local error string --------------------------------------------------
 void set_error(const char *fmt, ...);
 int cuda_fail(cudaError_t e, const char *what);

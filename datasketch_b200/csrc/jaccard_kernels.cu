@@ -46,6 +46,9 @@ __global__ void __launch_bounds__(256) jaccard_pairs_kernel(const uint32_t *__re
 // CTA tile: kTQ = 64 query rows x kTD = 128 database rows per step; 128 threads, thread <-> 8 queries x
 // 8 database rows (64 counters in registers).  Both tiles are staged TRANSPOSED in shared memory
 // ([position][row]) so a thread reads its 8 + 8 values of one signature position with four LDS.128.
+// The query tile is staged whole, once per query tile, when it fits a block's 227 KB of shared memory
+// (K <= 736); above that (WHOLE_Q = false) it goes through shared memory kKc positions at a time next to
+// the database chunk, a footprint of 49 KB whatever K, so every num_perm the API accepts runs.
 // After a database tile, counts above the query's current k-th best are inserted into the query's
 // sorted list in shared memory (ties keep the lower database index because tiles arrive in index
 // order and insertion requires a strictly larger count than the k-th entry ... or an unfilled slot).
@@ -61,12 +64,13 @@ struct TopkParams {
     int64_t *out_idx;     // [nq, topk]  (-1 = no such row)
 };
 
+template <bool WHOLE_Q>
 __global__ void __launch_bounds__(kTopThreads) jaccard_topk_kernel(const TopkParams p) {
     DSK_DYNAMIC_SMEM_T(uint32_t, sm, 16);
     const int K = p.k;
     const int kpad = (K + kKc - 1) / kKc * kKc;
-    uint32_t *sQ = sm;                              // [kpad][kTQ]
-    uint32_t *sD = sQ + (size_t)kpad * kTQ;         // [kKc][kTD]
+    uint32_t *sQ = sm;                                              // [kpad][kTQ] (WHOLE_Q) or [kKc][kTQ]
+    uint32_t *sD = sQ + (size_t)(WHOLE_Q ? kpad : kKc) * kTQ;      // [kKc][kTD]
     int32_t *top_cnt = reinterpret_cast<int32_t *>(sD + kKc * kTD);   // [kTQ][topk]
     int64_t *top_idx = reinterpret_cast<int64_t *>(top_cnt + kTQ * kMaxTopK);  // [kTQ][topk]
     int *lock = reinterpret_cast<int *>(top_idx + kTQ * kMaxTopK);    // [kTQ]
@@ -76,20 +80,23 @@ __global__ void __launch_bounds__(kTopThreads) jaccard_topk_kernel(const TopkPar
     const int tid = threadIdx.x;
     const int qg = tid >> 4, dg = tid & 15;         // 8 query groups x 16 database groups
     const int topk = p.topk;
+    const bool qvec = (K & 3) == 0 && (reinterpret_cast<uintptr_t>(p.q) & 15) == 0;   // the API checks only d_db's alignment
 
     for (int64_t qt = blockIdx.x; qt * kTQ < p.nq; qt += gridDim.x) {
         const int64_t q0 = qt * kTQ;
         __syncthreads();
         for (int i = tid; i < kTQ * kMaxTopK; i += kTopThreads) { top_cnt[i] = -1; top_idx[i] = -1; }
         for (int i = tid; i < kTQ; i += kTopThreads) { lock[i] = 0; thr[i] = -1; kidx[i] = -1; }
-        // query tile, transposed; rows / positions beyond the data are filled so they never match
-        for (int e = tid; e < kTQ * kpad; e += kTopThreads) {
-            const int r = e / kpad, c = e - r * kpad;
-            uint32_t v = 0x51EDu + (uint32_t)c;           // padded positions never match: the db side uses ~filler
-            if (q0 + r < p.nq && c < K) v = __ldg(p.q + (q0 + r) * (int64_t)K + c);
-            sQ[(size_t)c * kTQ + r] = v;
+        if (WHOLE_Q) {
+            // query tile, transposed; rows / positions beyond the data are filled so they never match
+            for (int e = tid; e < kTQ * kpad; e += kTopThreads) {
+                const int r = e / kpad, c = e - r * kpad;
+                uint32_t v = 0x51EDu + (uint32_t)c;           // padded positions never match: the db side uses ~filler
+                if (q0 + r < p.nq && c < K) v = __ldg(p.q + (q0 + r) * (int64_t)K + c);
+                sQ[(size_t)c * kTQ + r] = v;
+            }
+            __syncthreads();
         }
-        __syncthreads();
 
         for (int64_t d0 = 0; d0 < p.n; d0 += kTD) {
             int cnt[8][8];
@@ -99,6 +106,27 @@ __global__ void __launch_bounds__(kTopThreads) jaccard_topk_kernel(const TopkPar
                 for (int b = 0; b < 8; ++b) cnt[a][b] = 0;
             for (int c0 = 0; c0 < kpad; c0 += kKc) {
                 __syncthreads();
+                // stage query chunk [kTQ rows][kKc positions] transposed: each task = (row, 8 positions); rows and
+                // positions beyond the data get a filler that the database side never holds at that position
+                for (int task = tid; !WHOLE_Q && task < kTQ * (kKc / 8); task += kTopThreads) {
+                    const int r = task % kTQ, seg = task / kTQ;
+                    const int64_t row = q0 + r;
+                    const int cb = c0 + seg * 8;
+                    uint32_t v[8];
+                    if (row < p.nq && qvec && cb + 8 <= K) {
+                        const uint4 x = __ldg(reinterpret_cast<const uint4 *>(p.q + row * (int64_t)K + cb));
+                        const uint4 y = __ldg(reinterpret_cast<const uint4 *>(p.q + row * (int64_t)K + cb + 4));
+                        v[0] = x.x; v[1] = x.y; v[2] = x.z; v[3] = x.w; v[4] = y.x; v[5] = y.y; v[6] = y.z; v[7] = y.w;
+                    } else {
+#pragma unroll
+                        for (int u = 0; u < 8; ++u) {
+                            v[u] = 0x51EDu + (uint32_t)(cb + u);
+                            if (row < p.nq && cb + u < K) v[u] = __ldg(p.q + row * (int64_t)K + cb + u);
+                        }
+                    }
+#pragma unroll
+                    for (int u = 0; u < 8; ++u) sQ[(seg * 8 + u) * kTQ + r] = v[u];
+                }
                 // stage database chunk [kTD rows][kKc positions] transposed: each task = (row, 8 positions)
                 for (int task = tid; task < kTD * (kKc / 8); task += kTopThreads) {
                     const int r = task % kTD, seg = task / kTD;
@@ -122,8 +150,9 @@ __global__ void __launch_bounds__(kTopThreads) jaccard_topk_kernel(const TopkPar
                 __syncthreads();
 #pragma unroll 4
                 for (int cc = 0; cc < kKc; ++cc) {
-                    const uint4 qa = *reinterpret_cast<const uint4 *>(sQ + (size_t)(c0 + cc) * kTQ + qg * 8);
-                    const uint4 qb = *reinterpret_cast<const uint4 *>(sQ + (size_t)(c0 + cc) * kTQ + qg * 8 + 4);
+                    const uint32_t *qrow = sQ + (size_t)((WHOLE_Q ? c0 : 0) + cc) * kTQ;
+                    const uint4 qa = *reinterpret_cast<const uint4 *>(qrow + qg * 8);
+                    const uint4 qb = *reinterpret_cast<const uint4 *>(qrow + qg * 8 + 4);
                     const uint4 da = *reinterpret_cast<const uint4 *>(sD + cc * kTD + dg * 8);
                     const uint4 db = *reinterpret_cast<const uint4 *>(sD + cc * kTD + dg * 8 + 4);
                     const uint32_t qv[8] = {qa.x, qa.y, qa.z, qa.w, qb.x, qb.y, qb.z, qb.w};
@@ -372,18 +401,31 @@ __global__ void __launch_bounds__(kTopThreads) jaccard_topk_pf_kernel(const Topk
     }
 }
 
-// workspace of the prefilter path: the bit planes of both matrices (0 = the path does not apply: K < 32 or K > 512)
+// dynamic shared memory of jaccard_topk_pf_kernel: both tiles' bit planes, the per-query lists and the candidate queue
+size_t jaccard_topk_pf_smem(int k) {
+    const int words = (k + 31) / 32;
+    return (size_t)kPfB * words * (kTQ + kTD) * 4 + (size_t)kTQ * kMaxTopK * (4 + 8) + (size_t)kTQ * 16 + 16 +
+           (size_t)kTQ * kTD * 2;
+}
+
+// the prefilter needs K >= 32 to pay off and its planes must fit a block's shared memory (K <= 480)
+static bool jaccard_topk_pf_applies(int k) { return k >= 32 && jaccard_topk_pf_smem(k) <= kMaxDynamicSmemPerBlock; }
+
+// workspace of the prefilter path: the bit planes of both matrices (0 = the path does not apply)
 size_t jaccard_topk_workspace_bytes(int64_t nq, int64_t n, int k) {
-    if (k < 32 || k > 512 || n < 4 * kTD) return 0;
+    if (!jaccard_topk_pf_applies(k) || n < 4 * kTD) return 0;
     const int words = (k + 31) / 32;
     const size_t qt = (size_t)((nq + kTQ - 1) / kTQ), dt = (size_t)((n + kTD - 1) / kTD);
     return (qt * kTQ + dt * kTD) * (size_t)kPfB * words * sizeof(uint32_t);
 }
 
+// K whose planes do not fit (K > 480) runs the exact kernel instead; the workspace is then not touched
 cudaError_t launch_jaccard_topk_pf(const uint32_t *q, int64_t nq, const uint32_t *db, int64_t n, int k, int topk,
                                    int64_t self_base, int32_t *out_cnt, int64_t *out_idx, void *workspace, int sm_count,
                                    cudaStream_t s) {
     if (nq <= 0) return cudaSuccess;
+    if (jaccard_topk_pf_smem(k) > kMaxDynamicSmemPerBlock)
+        return launch_jaccard_topk(q, nq, db, n, k, topk, self_base, out_cnt, out_idx, sm_count, s);
     const int words = (k + 31) / 32;
     const size_t qt = (size_t)((nq + kTQ - 1) / kTQ);
     uint32_t *qpl = static_cast<uint32_t *>(workspace);
@@ -394,8 +436,7 @@ cudaError_t launch_jaccard_topk_pf(const uint32_t *q, int64_t nq, const uint32_t
     TopkPfParams p;
     p.q = q; p.db = db; p.qpl = qpl; p.dpl = dpl; p.nq = nq; p.n = n; p.k = k; p.words = words; p.topk = topk;
     p.self_base = self_base; p.out_cnt = out_cnt; p.out_idx = out_idx;
-    const size_t smem = (size_t)kPfB * words * (kTQ + kTD) * 4 + (size_t)kTQ * kMaxTopK * (4 + 8) + (size_t)kTQ * 16 + 16 +
-                        (size_t)kTQ * kTD * 2;
+    const size_t smem = jaccard_topk_pf_smem(k);
     cudaError_t e = cudaFuncSetAttribute(jaccard_topk_pf_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     int64_t grid = (nq + kTQ - 1) / kTQ;
@@ -404,9 +445,11 @@ cudaError_t launch_jaccard_topk_pf(const uint32_t *q, int64_t nq, const uint32_t
     return cudaGetLastError();
 }
 
-size_t jaccard_topk_smem(int k) {
+// dynamic shared memory of jaccard_topk_kernel: the query tile (whole, or one kKc chunk), the database chunk, the lists
+size_t jaccard_topk_smem(int k, bool whole_q) {
     const int kpad = (k + kKc - 1) / kKc * kKc;
-    return (size_t)kpad * kTQ * 4 + (size_t)kKc * kTD * 4 + (size_t)kTQ * kMaxTopK * (4 + 8) + (size_t)kTQ * 16;
+    return (size_t)(whole_q ? kpad : kKc) * kTQ * 4 + (size_t)kKc * kTD * 4 + (size_t)kTQ * kMaxTopK * (4 + 8) +
+           (size_t)kTQ * 16;
 }
 
 cudaError_t launch_jaccard_topk(const uint32_t *q, int64_t nq, const uint32_t *db, int64_t n, int k, int topk,
@@ -415,12 +458,16 @@ cudaError_t launch_jaccard_topk(const uint32_t *q, int64_t nq, const uint32_t *d
     TopkParams p;
     p.q = q; p.db = db; p.nq = nq; p.n = n; p.k = k; p.topk = topk; p.self_base = self_base;
     p.out_cnt = out_cnt; p.out_idx = out_idx;
-    const size_t smem = jaccard_topk_smem(k);
-    cudaError_t e = cudaFuncSetAttribute(jaccard_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const bool whole_q = jaccard_topk_smem(k, true) <= kMaxDynamicSmemPerBlock;
+    const size_t smem = jaccard_topk_smem(k, whole_q);
+    cudaError_t e = whole_q
+        ? cudaFuncSetAttribute(jaccard_topk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+        : cudaFuncSetAttribute(jaccard_topk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     int64_t grid = (nq + kTQ - 1) / kTQ;
     if (grid > (int64_t)sm_count * 3) grid = (int64_t)sm_count * 3;
-    DSK_LAUNCH(jaccard_topk_kernel, (unsigned)grid, kTopThreads, smem, s, p);
+    if (whole_q) DSK_LAUNCH((jaccard_topk_kernel<true>), (unsigned)grid, kTopThreads, smem, s, p);
+    else DSK_LAUNCH((jaccard_topk_kernel<false>), (unsigned)grid, kTopThreads, smem, s, p);
     return cudaGetLastError();
 }
 

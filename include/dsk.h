@@ -244,13 +244,14 @@ DSK_API int dsk_jaccard_pairs(const uint32_t *d_sig, int64_t n_rows, int num_per
                               const int64_t *d_j, int64_t m, int32_t *d_count, void *stream);
 
 /* All-pairs top-k: for each of nq query rows, the `topk` (<= 32) rows of the [n, num_perm]
- * database with the most equal positions, best first; ties -> lower database index.  If
+ * (num_perm <= 4096) database with the most equal positions, best first; ties -> lower database index.  If
  * self_base >= 0, query i is database row self_base + i and is excluded from its own list.
  * d_cnt [nq, topk] int32 counts (jaccard = cnt / num_perm), d_idx [nq, topk] int64 (-1 pads). */
 DSK_API int dsk_jaccard_topk(const uint32_t *d_q, int64_t nq, const uint32_t *d_db, int64_t n, int num_perm, int topk,
                              int64_t self_base, int32_t *d_cnt, int64_t *d_idx, void *stream);
 /* Same result, ~3x fewer ALU ops: with a caller-provided workspace (16-byte aligned, >= dsk_jaccard_topk_workspace_size()
- * bytes -- 0 means the prefilter does not apply and the call behaves like dsk_jaccard_topk) both matrices are first reduced
+ * bytes -- 0 means the prefilter does not apply and the call behaves like dsk_jaccard_topk: num_perm < 32, num_perm > 480
+ * (the fingerprint planes would not fit a block's shared memory) or n < 512) both matrices are first reduced
  * to bit-sliced 16-bit fingerprints; a pair reaches the exact count only if the fingerprint agreement -- an upper bound of
  * the number of equal positions -- could still enter the query's list.  Lists are identical to dsk_jaccard_topk's. */
 DSK_API size_t dsk_jaccard_topk_workspace_size(int64_t nq, int64_t n, int num_perm);

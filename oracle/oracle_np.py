@@ -131,6 +131,39 @@ def jaccard(hv1: np.ndarray, hv2: np.ndarray) -> float:
     return float(np.count_nonzero(hv1 == hv2)) / float(len(hv1))
 
 
+def jaccard_topk(q: np.ndarray, db: np.ndarray, topk: int, self_base: int = -1) -> Tuple[np.ndarray, np.ndarray]:
+    """Brute-force top-k by ``jaccard`` over two signature matrices, as counts of equal positions.
+
+    Per query row: the ``topk`` database rows with the most equal positions, count descending then
+    index ascending; ``self_base >= 0`` leaves database row ``self_base + i`` out of query i's list.
+    Returns ``(count, index)``, both int64 [Q, topk], -1 where the database has fewer rows.  Counts
+    are int64 sums of boolean compares, taken a few queries at a time to bound memory.
+    """
+    q, db = np.asarray(q), np.asarray(db)
+    nq, n, k = len(q), len(db), q.shape[1]
+    out_c = np.full((nq, topk), -1, np.int64)
+    out_i = np.full((nq, topk), -1, np.int64)
+    if nq == 0 or n == 0:
+        return out_c, out_i
+    excluded = np.int64((k + 1) * (n + 1))          # ranks after every real key
+    step = max(1, (1 << 25) // max(1, n * k))
+    for s in range(0, nq, step):
+        blk = q[s:s + step]
+        cnt = (blk[:, None, :] == db[None, :, :]).sum(axis=2, dtype=np.int64)
+        key = (k - cnt) * (n + 1) + np.arange(n, dtype=np.int64)[None, :]      # count desc, then index asc
+        if self_base >= 0:
+            rows = self_base + np.arange(s, s + len(blk))
+            hit = rows < n
+            key[np.nonzero(hit)[0], rows[hit]] = excluded
+        m = min(topk, n)
+        order = np.argsort(key, axis=1, kind="stable")[:, :m]
+        sel_key = np.take_along_axis(key, order, axis=1)
+        keep = sel_key != excluded
+        out_i[s:s + len(blk), :m] = np.where(keep, order, -1)
+        out_c[s:s + len(blk), :m] = np.where(keep, np.take_along_axis(cnt, order, axis=1), -1)
+    return out_c, out_i
+
+
 def merge(hv1: np.ndarray, hv2: np.ndarray) -> np.ndarray:
     """Element-wise min (datasketch/minhash.py:359)."""
     return np.minimum(hv2, hv1)

@@ -15,6 +15,8 @@
 #include <math.h>
 
 #include <atomic>
+#include <map>
+#include <mutex>
 
 #define __global__
 #define __device__
@@ -27,11 +29,35 @@
 typedef int cudaError_t;
 typedef void *cudaStream_t;
 enum { cudaSuccess = 0 };
+enum { cudaErrorInvalidValue = 1, cudaErrorMemoryAllocation = 2, cudaErrorInsufficientDriver = 35, cudaErrorNoDevice = 100 };
 enum { cudaFuncAttributeMaxDynamicSharedMemorySize = 8 };
-static inline cudaError_t cudaGetLastError() { return cudaSuccess; }
-static inline cudaError_t cudaMemsetAsync(void *p, int v, size_t n, cudaStream_t) { memset(p, v, n); return cudaSuccess; }
+
+// ---- shared-memory limits of an sm_100 block, enforced like the driver does: a launch may use 48 KB of dynamic shared
+// memory, or up to what cudaFuncSetAttribute raised the kernel's limit to, and that may not exceed 227 KB.  A launch
+// over its limit runs nothing and leaves the error for cudaGetLastError.
+constexpr size_t kEmuSmemDefault = 48 << 10, kEmuSmemOptin = 232448;
+static inline cudaError_t &emu_last_error() { static thread_local cudaError_t e = cudaSuccess; return e; }
+static inline cudaError_t cudaGetLastError() {
+    const cudaError_t e = emu_last_error();
+    emu_last_error() = cudaSuccess;
+    return e;
+}
+static inline std::map<const void *, size_t> &emu_smem_limits() { static std::map<const void *, size_t> m; return m; }
+static inline std::mutex &emu_smem_mu() { static std::mutex m; return m; }
 template <typename F>
-static inline cudaError_t cudaFuncSetAttribute(F, int, int) { return cudaSuccess; }
+static inline cudaError_t cudaFuncSetAttribute(F kernel, int attr, int value) {
+    if (attr != cudaFuncAttributeMaxDynamicSharedMemorySize) return cudaSuccess;
+    if (value < 0 || (size_t)value > kEmuSmemOptin) return cudaErrorInvalidValue;
+    std::lock_guard<std::mutex> lk(emu_smem_mu());
+    emu_smem_limits()[reinterpret_cast<const void *>(kernel)] = (size_t)value;
+    return cudaSuccess;
+}
+static inline size_t emu_smem_limit(const void *kernel) {
+    std::lock_guard<std::mutex> lk(emu_smem_mu());
+    const auto it = emu_smem_limits().find(kernel);
+    return it == emu_smem_limits().end() ? kEmuSmemDefault : it->second;
+}
+static inline cudaError_t cudaMemsetAsync(void *p, int v, size_t n, cudaStream_t) { memset(p, v, n); return cudaSuccess; }
 
 struct uint3e { unsigned x, y, z; };
 struct uint2 { uint32_t x, y; };
@@ -99,9 +125,8 @@ static inline unsigned long long atomicExch(unsigned long long *p, unsigned long
 static inline void __threadfence_block() { __atomic_thread_fence(__ATOMIC_SEQ_CST); }
 
 // ---- CUDA runtime, synchronous and on host memory: "device" pointers are host pointers, one fake device with two SMs
-enum { cudaErrorInvalidValue = 1, cudaErrorMemoryAllocation = 2, cudaErrorInsufficientDriver = 35, cudaErrorNoDevice = 100 };
 enum { cudaStreamNonBlocking = 1 };
-struct cudaDeviceProp { int multiProcessorCount, major, minor; size_t totalGlobalMem; char name[64]; };
+struct cudaDeviceProp { int multiProcessorCount, major, minor; size_t totalGlobalMem, sharedMemPerBlockOptin; char name[64]; };
 static inline const char *cudaGetErrorString(cudaError_t e) { return e == cudaSuccess ? "no error" : "emulated CUDA error"; }
 static inline cudaError_t cudaGetDeviceCount(int *n) { *n = 1; return cudaSuccess; }
 static inline cudaError_t cudaGetDevice(int *d) { *d = 0; return cudaSuccess; }
@@ -109,6 +134,7 @@ static inline cudaError_t cudaSetDevice(int d) { return d == 0 ? cudaSuccess : c
 static inline cudaError_t cudaGetDeviceProperties(cudaDeviceProp *p, int) {
     memset(p, 0, sizeof(*p));
     p->multiProcessorCount = 2; p->major = 10; p->minor = 0; p->totalGlobalMem = (size_t)8 << 30;
+    p->sharedMemPerBlockOptin = kEmuSmemOptin;
     strcpy(p->name, "emulated sm_100 (host threads)");
     return cudaSuccess;
 }
@@ -232,6 +258,10 @@ static inline int __any_sync(unsigned, int pred) { return emu_ballot(pred != 0) 
 #include <vector>
 template <typename... KArgs, typename... Args>
 static inline void emu_launch(void (*kernel)(KArgs...), dim3 grid, unsigned block_threads, size_t smem_bytes, Args... args) {
+    if (smem_bytes > emu_smem_limit(reinterpret_cast<const void *>(kernel))) {
+        emu_last_error() = cudaErrorInvalidValue;
+        return;
+    }
     std::tuple<KArgs...> kargs(static_cast<KArgs>(args)...);
     const unsigned nwarps = (block_threads + 31) / 32;
     std::vector<EmuWarp> warps(nwarps);

@@ -135,20 +135,6 @@ def test_jaccard_pairs_matches_golden_objects(dsk, golden):
     assert dsk.codec.jaccard_pairs(sig, [0], [1])[0] == float(g["j_jaccard"])
 
 
-def _topk_oracle(q, db, topk, self_base):
-    out_c, out_i = [], []
-    for i, row in enumerate(q):
-        cnt = (db == row[None, :]).sum(axis=1).astype(np.int64)
-        order = np.lexsort((np.arange(len(db)), -cnt))          # count desc, index asc
-        if self_base >= 0:
-            order = order[order != self_base + i]
-        order = order[:topk]
-        c = np.full(topk, -1, np.int64); ix = np.full(topk, -1, np.int64)
-        c[:len(order)] = cnt[order]; ix[:len(order)] = order
-        out_c.append(c); out_i.append(ix)
-    return np.stack(out_c), np.stack(out_i)
-
-
 @pytest.mark.parametrize("k,n,nq,topk,self_base", [(128, 1000, 150, 10, 0), (100, 333, 70, 5, -1), (128, 7, 7, 10, 0),
                                                     (64, 2000, 65, 32, 500), (256, 300, 10, 1, -1)])
 def test_jaccard_topk_vs_oracle(dsk, k, n, nq, topk, self_base):
@@ -161,7 +147,7 @@ def test_jaccard_topk_vs_oracle(dsk, k, n, nq, topk, self_base):
     else:
         q = rs.randint(0, 3, size=(nq, k)).astype(np.uint32)
     jac, idx = dsk.codec.jaccard_topk(q, db, topk=topk, self_base=self_base)
-    wc, wi = _topk_oracle(q, db, topk, self_base)
+    wc, wi = o.jaccard_topk(q, db, topk, self_base)
     assert np.array_equal(idx, wi)
     assert np.array_equal(jac, np.where(wc >= 0, wc, 0) / float(k))
 
@@ -176,7 +162,7 @@ def test_jaccard_topk_random_signatures_finds_planted_pairs(dsk):
         db[i + 1, rs.choice(k, 10, replace=False)] = 7
     q = db[:512]
     jac, idx = dsk.codec.jaccard_topk(q, db, topk=10, self_base=0)
-    wc, wi = _topk_oracle(q[:64], db, 10, 0)
+    wc, wi = o.jaccard_topk(q[:64], db, 10, 0)
     assert np.array_equal(idx[:64], wi)
     assert all(idx[i, 0] == i + 1 for i in range(0, 512, 2)) and all(idx[i, 0] == i - 1 for i in range(1, 512, 2))
     assert (jac[:, 0] >= 118 / 128).all() and (jac[:, 1] < 0.1).all()
@@ -189,7 +175,7 @@ def test_sharded_topk_single_process_equals_kernel(dsk):
     import torch
     d = torch.from_numpy(sig.view(np.int32)).cuda()
     cnt, idx = dsk.distributed.sharded_jaccard_topk(d, topk=7)
-    wc, wi = _topk_oracle(sig, sig, 7, 0)
+    wc, wi = o.jaccard_topk(sig, sig, 7, 0)
     assert np.array_equal(idx.cpu().numpy(), wi) and np.array_equal(cnt.cpu().numpy(), wc)
     full, base, counts = dsk.distributed.gather_signature_blocks(d)
     assert full is d and base == 0 and counts == [500]

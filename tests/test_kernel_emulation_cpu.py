@@ -431,11 +431,14 @@ def test_jaccard_pairs_and_topk_kernels(emu):
         assert np.array_equal(oc_idx[i], order) and np.array_equal(oc_cnt[i], c[order])
 
 
-@pytest.mark.parametrize("k,n,nq,topk,vals", [(64, 200, 66, 5, 3), (128, 260, 40, 10, 1 << 32), (100, 257, 40, 7, 50), (32, 140, 10, 32, 2)])
+@pytest.mark.parametrize("k,n,nq,topk,vals", [(64, 200, 66, 5, 3), (128, 260, 40, 10, 1 << 32), (100, 257, 40, 7, 50), (32, 140, 10, 32, 2),
+                                              (512, 140, 10, 10, 2), (1024, 140, 10, 32, 3)])
 def test_topk_with_fingerprint_prefilter_equals_exact(emu, k, n, nq, topk, vals):
     """jaccard_topk_pf_kernel: bit-sliced 16-bit fingerprints give an upper bound of the match count; only pairs whose bound
     could still enter the list are counted exactly -- the lists must equal a brute-force ranking (and the exact kernel's):
-    heavy ties (3 distinct values), no similarity at all (random 32-bit), K not a multiple of 32, topk = 32."""
+    heavy ties (3 distinct values), no similarity at all (random 32-bit), K not a multiple of 32, topk = 32.  At K = 512 and
+    1024 the prefilter's planes exceed a block's 227 KB of shared memory (the emulation enforces the limit): the launcher
+    must run the exact kernel, whose footprint does not grow with K."""
     lib = emu.lib
     rs = np.random.RandomState(k + n)
     db = rs.randint(0, vals, size=(n, k), dtype=np.uint64).astype(np.uint32)
